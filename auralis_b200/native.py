@@ -325,8 +325,13 @@ class NativeEngine:
         return out
 
     def run_batch(self, jobs, timeout_s: float = 600.0, want_wav: bool = True, want_latents: bool = False):
-        """jobs: iterable of (seq_id, text_ids, speaker_slot, Sampling).  Returns {seq_id: (result, tokens, wav, lat)}."""
+        """jobs: iterable of (seq_id, text_ids, speaker_slot, Sampling).  Returns {seq_id: (result, tokens, wav, lat)}.
+        want_wav: True / False, or a set of seq ids whose waveforms are copied out (the others' wav is None)."""
         import time
+        wav_ids = None if isinstance(want_wav, bool) else frozenset(want_wav)
+
+        def wants_wav(sid):
+            return want_wav if wav_ids is None else sid in wav_ids
         n = 0
         # batch submit: the scheduler admits nothing until the whole batch is queued, so admission waves (and with
         # them which chunks finish together and share a vocoder launch) do not depend on host timing
@@ -349,10 +354,10 @@ class NativeEngine:
                 self.lib.xtts_fetch(self.h, r.seq_id, None, None, None)      # releases the failed chunk's native buffers
                 raise NativeError(f"sequence {r.seq_id} failed ({r.status}): {self.lib.xtts_last_error().decode()}")
             if r.status > 0:                 # partial piece (Sampling.early_tokens): kept, in order, next to the final result
-                ptoks, pwav, _ = self.fetch(r, want_wav, False)
+                ptoks, pwav, _ = self.fetch(r, wants_wav(r.seq_id), False)
                 partials.setdefault(r.seq_id, []).append((r, ptoks, pwav))
                 continue
-            toks, wav, lat = self.fetch(r, want_wav, want_latents)
+            toks, wav, lat = self.fetch(r, wants_wav(r.seq_id), want_latents)
             out[r.seq_id] = (r, toks, wav, lat)
         self.last_partials = partials        # {seq_id: [(result, tokens, wav), ...]} of the batch just run, oldest first
         return out

@@ -36,6 +36,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 SEED = 1234
+DUMP_WAV_CHUNKS = 16            # --dump-outputs: a full step's waveforms are ~440 MB, 16 chunks ~40 MB
 WORDS = ("the of and to in is that it was for on are as with his they at be this from have or by one had not but what "
          "all were when we there can an your which their said if do will each about how up out them then she many some "
          "so these would other into has more her two like him see time could no make than first been its who now people "
@@ -117,6 +118,26 @@ class ClockSampler:
                 "power_w_max": max(float(r[2]) for r in rows), "samples": len(rows)}
 
 
+def dump_outputs(out_dir: str, res: dict) -> None:
+    """Writes one step's results {seq_id: (result, tokens, wav or None, _)} as float32 .npy files: tokens [chunks, max
+    tokens] padded with -1, n_tokens / n_samples [chunks], the fetched waveforms [k, max samples] zero-padded and their
+    seq ids [k].  Every value is an integer below 2^24 or a float32 sample, so float32 holds it exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    sids = sorted(res)
+    n_tok = np.array([res[s][0].n_tokens for s in sids], np.float32)
+    toks = np.full((len(sids), max(1, int(n_tok.max(initial=0)))), -1, np.float32)
+    for i, s in enumerate(sids):
+        toks[i, : len(res[s][1])] = res[s][1]
+    wav_ids = [s for s in sids if res[s][2] is not None]
+    wavs = np.zeros((len(wav_ids), max([res[s][2].size for s in wav_ids], default=0)), np.float32)
+    for i, s in enumerate(wav_ids):
+        wavs[i, : res[s][2].size] = res[s][2]
+    arrays = {"tokens": toks, "n_tokens": n_tok, "n_samples": np.array([res[s][0].n_samples for s in sids], np.float32),
+              "waveforms": wavs, "waveform_seq_ids": np.array(wav_ids, np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # =====================================================================================================
 def cpu_reference_sample(dims, state, n_threads: int, chunks=None, n_chunks: int = 8, max_tokens: int = 48) -> dict:
     """One TIMED pass of the reference's CPU path (the oracle port, fp32 torch ops, all host threads) over a bounded sample
@@ -161,7 +182,7 @@ def cpu_reference_sample(dims, state, n_threads: int, chunks=None, n_chunks: int
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=int, default=2, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--precision", default="fp16", choices=["bf16", "fp16", "fp32"],
@@ -176,7 +197,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra arms (ragged lengths, cfg3 time-to-first-audio, fp32 parity mode, strong scaling)")
     ap.add_argument("--sweep", action="store_true", help="option sweeps only: skip the e2e arm and the CPU baseline (the line says so; not a headline run)")
     ap.add_argument("--small", action="store_true", help="tiny geometry (plumbing check only; not a valid bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (B200 arm: rank 0's tokens of every chunk "
+                         f"and the waveforms of {DUMP_WAV_CHUNKS} chunks picked with a fixed seed) to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the B200 arm")
 
     import torch
     from auralis_b200.config import XTTSDims
@@ -249,8 +277,15 @@ def main():
     n_chunks = sum(len(c) for c in reqs_chunks)
     max_tok = min(args.max_tokens, dims.gpt.max_audio_tokens)
 
-    def device_step(step_idx: int, lengths=None, chunk_lists=None):
-        """lengths: per-chunk max_tokens (the ragged arm); chunk_lists: another request set (the strong-scaling arm)"""
+    # --dump-outputs: the last timed step copies these chunks' waveforms out of HBM (the others stay there, as in every step)
+    dump_wav_ids = set()
+    if args.dump_outputs:
+        dump_wav_ids = set(np.random.RandomState(SEED).choice(n_chunks, min(DUMP_WAV_CHUNKS, n_chunks), replace=False).tolist())
+    dumped = {}
+
+    def device_step(step_idx: int, lengths=None, chunk_lists=None, want_wav=False):
+        """lengths: per-chunk max_tokens (the ragged arm); chunk_lists: another request set (the strong-scaling arm);
+        want_wav: seq ids whose waveforms are fetched, the results are then kept in `dumped`"""
         jobs, sid = [], 0
         for ri, chunks in enumerate(chunk_lists if chunk_lists is not None else reqs_chunks):
             for ci, ids in enumerate(chunks):
@@ -259,8 +294,14 @@ def main():
                                      stop_token=dims.gpt.stop_audio_token, seed=SEED + step_idx, seq_seed=sid, vocode=True)
                 jobs.append((sid, ids, spk_slots[ri % 4], sp))
                 sid += 1
-        res = eng.run_batch_direct(jobs, timeout_s=900, want_wav=False)
+        res = eng.run_batch_direct(jobs, timeout_s=900, want_wav=want_wav)
+        if want_wav:
+            dumped.clear()
+            dumped.update(res)
         return sum(r.n_samples for (r, _, _, _) in res.values()), sum(r.n_tokens for (r, _, _, _) in res.values())
+
+    def timed_device_step(step_idx: int):
+        return device_step(step_idx, want_wav=dump_wav_ids if step_idx == args.steps - 1 else False)
 
     def e2e_step(step_idx: int):
         reqs = [TTSRequest(text=t, speaker_files=spk_bytes[i % 4], language="en", temperature=0.75, top_p=0.85, top_k=50,
@@ -336,8 +377,10 @@ def main():
     ne.set_option("reset_stats", 0)
     if sampler:
         sampler.start()
-    dt_dev, wall_dev, acc_dev, span = timed(device_step, 0, args.steps)
+    dt_dev, wall_dev, acc_dev, span = timed(timed_device_step, 0, args.steps)
     clocks = sampler.stop(*span) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
     st = ne.stats()
     samples_dev = sum(a[0] for a in acc_dev)
     tokens_dev = sum(a[1] for a in acc_dev)

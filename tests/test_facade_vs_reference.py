@@ -1,5 +1,6 @@
-"""CPU, container only: the public façade (`auralis_b200.TTS` / `TTSRequest` / `TTSOutput`) against the REFERENCE's own
-classes (`auralis.core.tts.TTS` etc., imported unmodified by oracle/ref_facade.py).  Both are driven by the same fake engine
+"""CPU: the public façade (`auralis_b200.TTS` / `TTSRequest` / `TTSOutput`) against what the REFERENCE's own classes
+(`auralis.core.tts.TTS` etc., imported unmodified by oracle/ref_facade.py) returned, stored in
+tests/golden/facade_vs_reference.npz (tests/reference_records.py).  Both are driven by the same fake engine
 — per chunk one waveform whose values encode (request text length, chunk index), earlier chunks finishing LATER — and must
 return the same audio in the same order for: one-shot generation, streaming, several chunks, the 100 000-character request
 split (`split_requests`), a prepared speaker (`prepare_for_streaming_generation`), the async API, and a failing chunk."""
@@ -11,8 +12,10 @@ import pytest
 
 import auralis_b200 as ours
 from oracle import ref_import
+from reference_records import Records, sample
 
-pytestmark = [pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted"), pytest.mark.timeout(120)]
+pytestmark = pytest.mark.timeout(120)
+rec = Records("facade_vs_reference")
 
 
 def make_engine(ns_output, cond_config, fail_at=None):
@@ -54,61 +57,68 @@ def make_engine(ns_output, cond_config, fail_at=None):
     return Engine()
 
 
-@pytest.fixture(scope="module")
-def ref():
+def _ref():
     from oracle import ref_facade
     return ref_facade.load()
 
 
-def _sides(ref, **kw):
+def _side(which, conc=4, **kw):
+    """(TTS driving the fake engine, TTSRequest class) of the reference's façade ("ref") or ours"""
+    if which == "ref":
+        import importlib
+        ref = _ref()
+        RefCC = importlib.import_module("auralis.models.base").ConditioningConfig
+        r = ref.TTS(scheduler_max_concurrency=conc)
+        r._ensure_event_loop()
+        r.tts_engine = make_engine(ref.TTSOutput, RefCC(speaker_embeddings=True, gpt_like_decoder_conditioning=True), **kw)
+        return r, ref.TTSRequest
     from auralis_b200.base import ConditioningConfig as OursCC
-    import importlib
-    RefCC = importlib.import_module("auralis.models.base").ConditioningConfig
-    r = ref.TTS(scheduler_max_concurrency=4)
-    r._ensure_event_loop()
-    r.tts_engine = make_engine(ref.TTSOutput, RefCC(speaker_embeddings=True, gpt_like_decoder_conditioning=True), **kw)
-    o = ours.TTS(scheduler_max_concurrency=4).from_engine(make_engine(ours.TTSOutput, OursCC(True, True), **kw))
-    return (r, ref.TTSRequest), (o, ours.TTSRequest)
+    return ours.TTS(scheduler_max_concurrency=conc).from_engine(make_engine(ours.TTSOutput, OursCC(True, True), **kw)), ours.TTSRequest
+
+
+def _both(key, body, **kw):
+    """-> (what body(tts, Req) returned on the reference's façade, as recorded; what it returns on ours)"""
+    return rec(key, lambda: body(*_side("ref", **kw))), body(*_side("ours", **kw))
 
 
 @pytest.mark.parametrize("n_chars", [5, 55, 200])
-def test_generate_speech_same_audio(ref, n_chars):
-    res = []
-    for tts, Req in _sides(ref):
+def test_generate_speech_same_audio(n_chars):
+    def body(tts, Req):
         out = tts.generate_speech(Req(text="x" * n_chars, speaker_files=["s.wav"], language="en"))
-        res.append((np.asarray(out.array), out.sample_rate))
+        return np.asarray(out.array), out.sample_rate
+    res = _both(f"generate_speech[{n_chars}]", body)
     np.testing.assert_array_equal(res[0][0], res[1][0])
     assert res[0][1] == res[1][1] == 24000
 
 
-def test_streaming_same_chunks_in_same_order(ref):
-    res = []
-    for tts, Req in _sides(ref):
+def test_streaming_same_chunks_in_same_order():
+    def body(tts, Req):
         chunks = list(tts.generate_speech(Req(text="y" * 64, speaker_files=["s.wav"], language="en", stream=True)))
-        res.append([(np.asarray(c.array).tolist(), c.token_length) for c in chunks])
+        return [(np.asarray(c.array).tolist(), c.token_length) for c in chunks]
+    res = _both("streaming", body)
     assert res[0] == res[1] and len(res[0]) == 6
 
 
-def test_long_request_is_split_like_the_reference(ref):
-    res = []
-    for tts, Req in _sides(ref):
+def test_long_request_is_split_like_the_reference():
+    def split(tts, Req):
         req = Req(text="z" * 250_035, speaker_files=["s.wav"], language="en")
         parts = tts.split_requests(req, max_length=100_000)
-        res.append([len(p.text) for p in parts])
         assert len({p.request_id for p in parts}) == len(parts)
+        return [len(p.text) for p in parts]
+    res = _both("split_requests", split)
     assert res[0] == res[1] == [100_000, 100_000, 50_035]
+
     # and the audio of a (smaller) split request is the concatenation of its parts, in order
-    res = []
-    for tts, Req in _sides(ref):
+    def audio(tts, Req):
         tts.split_requests = lambda request, max_length=100000, _f=type(tts).split_requests: _f(request, 30)
         out = tts.generate_speech(Req(text="w" * 75, speaker_files=["s.wav"], language="en"))
-        res.append(np.asarray(out.array))
+        return np.asarray(out.array)
+    res = _both("split_request_audio", audio)
     np.testing.assert_array_equal(res[0], res[1])
 
 
-def test_prepared_speaker_and_async_api(ref):
-    res = []
-    for tts, Req in _sides(ref):
+def test_prepared_speaker_and_async_api():
+    def body(tts, Req):
         base = Req(text="q" * 40, speaker_files=["s.wav"], language="en")
         fn = tts.loop.run_until_complete(tts.prepare_for_streaming_generation(base))
         calls = tts.tts_engine.cond_calls
@@ -119,53 +129,61 @@ def test_prepared_speaker_and_async_api(ref):
                                                       context_partial_function=fn))
             b = [np.asarray(c.array).tolist() async for c in gen]
             return np.asarray(a.array).tolist(), b
-        res.append(tts.loop.run_until_complete(go()))
+        out = tts.loop.run_until_complete(go())
         assert tts.tts_engine.cond_calls == calls                  # the prepared conditioning is reused, not recomputed
+        return out
+    res = _both("prepared_speaker", body)
     assert res[0] == res[1]
 
 
-def test_failing_chunk_raises_the_same_error(ref):
-    errs = []
-    for tts, Req in _sides(ref, fail_at=1):
+def test_failing_chunk_raises_the_same_error():
+    def body(tts, Req):
         with pytest.raises(Exception) as ei:
             tts.generate_speech(Req(text="x" * 30, speaker_files=["s.wav"], language="en"))
-        errs.append((type(ei.value).__name__, str(ei.value)))
+        return type(ei.value).__name__, str(ei.value)
+    errs = _both("failing_chunk", body, fail_at=1)
     assert errs[0] == errs[1] == ("RuntimeError", "chunk 1 exploded")
 
 
-def test_request_defaults_and_validation_match(ref):
-    a = ref.TTSRequest(text="hi", speaker_files=["a.wav"])
-    b = ours.TTSRequest(text="hi", speaker_files=["a.wav"])
-    for f in ("temperature", "top_p", "top_k", "repetition_penalty", "length_penalty", "do_sample", "max_ref_length", "gpt_cond_len",
-              "gpt_cond_chunk_len", "stream", "enhance_speech", "load_sample_rate", "sound_norm_refs", "language"):
-        assert getattr(a, f) == getattr(b, f), f
-    for cls in (ref.TTSRequest, ours.TTSRequest):
+def test_request_defaults_and_validation_match():
+    def body(cls):
+        r = cls(text="hi", speaker_files=["a.wav"])
         with pytest.raises(ValueError):
             cls(text="hi", speaker_files=["a.wav"], language="klingon")
+        return {f: getattr(r, f) for f in ("temperature", "top_p", "top_k", "repetition_penalty", "length_penalty", "do_sample",
+                                           "max_ref_length", "gpt_cond_len", "gpt_cond_chunk_len", "stream", "enhance_speech",
+                                           "load_sample_rate", "sound_norm_refs", "language")}
+    want = rec("request_defaults", lambda: body(_ref().TTSRequest))
+    got = body(ours.TTSRequest)
+    for f in want:
+        assert got[f] == want[f], f
 
 
-def test_output_helpers_match(ref):
+def test_output_helpers_match():
     """TTSOutput: bytes constructor (int16 + fade-in), combine_outputs, pcm encodings, resample, get_info, from_tensor."""
     import torch
     rng = np.random.RandomState(1)
     x = (rng.rand(4800).astype(np.float32) * 1.9 - 0.95)
     pcm = (rng.randint(-30000, 30000, size=600)).astype(np.int16).tobytes()
-    sides = []
-    for Out in (ref.TTSOutput, ours.TTSOutput):
+
+    def body(Out):
         a, b, c = Out(array=x.copy()), Out(array=x[::-1].copy()), Out(array=pcm)
         comb = Out.combine_outputs([a, b, c])
         rs = a.resample(16000)
-        sides.append(dict(
+        side = dict(
             from_bytes=np.asarray(c.array), comb=np.asarray(comb.array), comb_sr=comb.sample_rate,
             pcm2=a.to_bytes("pcm", 2), pcm4=a.to_bytes("pcm", 4), pcm1=a.to_bytes("pcm", 1),
             rs=np.asarray(rs.array), rs_sr=rs.sample_rate, info=a.get_info(),
-            ft=np.asarray(Out.from_tensor(torch.from_numpy(x)[None], 22050).array), tensor=a.to_tensor().numpy()))
+            ft=np.asarray(Out.from_tensor(torch.from_numpy(x)[None], 22050).array), tensor=a.to_tensor().numpy())
         with pytest.raises(ValueError):
             a.to_bytes("ogg")
-    r, o = sides
+        return {k: sample(np.frombuffer(v, np.uint8) if isinstance(v, bytes) else v) if isinstance(v, (bytes, np.ndarray)) else v
+                for k, v in side.items()}
+    r, o = rec("output_helpers", lambda: body(_ref().TTSOutput)), body(ours.TTSOutput)
     for k in r:
-        if isinstance(r[k], np.ndarray):
-            np.testing.assert_array_equal(o[k], r[k], err_msg=k)
+        if isinstance(r[k], tuple) and isinstance(r[k][1], np.ndarray):       # sample() of an array or bytes
+            assert o[k][0] == r[k][0], k
+            np.testing.assert_array_equal(o[k][1], r[k][1], err_msg=k)
         else:
             assert o[k] == r[k], k
 
@@ -197,32 +215,31 @@ def test_load_audio_matches_the_reference_pipeline(tmp_path):
             nch, sr, raw = w.getnchannels(), w.getframerate(), w.readframes(w.getnframes())
         a = torch.from_numpy(np.frombuffer(raw, dtype="<i2").astype(np.float32) / 32768.0).reshape(-1, nch).t().contiguous()
         return a, sr
-    path = os.path.join(ref_import.REF_SRC, "auralis", "common", "utilities.py")
-    tree = ast.parse(open(path).read())
-    fn = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "load_audio"]
-    ns = {"torch": torch, "torchaudio": types.SimpleNamespace(load=fake_load, functional=torchaudio.functional)}
-    exec(compile(ast.Module(body=fn, type_ignores=[]), path, "exec"), ns)
+    def reference_load_audio(b):
+        path = os.path.join(ref_import.REF_SRC, "auralis", "common", "utilities.py")
+        tree = ast.parse(open(path).read())
+        fn = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "load_audio"]
+        ns = {"torch": torch, "torchaudio": types.SimpleNamespace(load=fake_load, functional=torchaudio.functional)}
+        exec(compile(ast.Module(body=fn, type_ignores=[]), path, "exec"), ns)
+        return ns["load_audio"](b, 22050)[0]
     for sr, nch in ((48000, 2), (22050, 1), (16000, 1), (44100, 2)):
         b = wav_bytes(sr, nch, seed=sr)
-        want = ns["load_audio"](b, 22050)[0].numpy()
+        shape, want = rec(f"load_audio[{sr},{nch}]", lambda: sample(reference_load_audio(b)))
         got = load_audio(b, 22050)
-        assert got.dtype == np.float32 and got.shape == want.shape
-        np.testing.assert_allclose(got, want, atol=1e-6, rtol=0)
+        assert got.dtype == np.float32 and got.shape == shape
+        np.testing.assert_allclose(sample(got)[1], want, atol=1e-6, rtol=0)
         f = tmp_path / f"a{sr}.wav"
         f.write_bytes(b)
-        np.testing.assert_allclose(load_audio(str(f), 22050), want, atol=1e-6, rtol=0)
+        np.testing.assert_allclose(load_audio(str(f), 22050), got, atol=1e-6, rtol=0)
     # IEEE-float WAV (what the reference's own TTSOutput.save writes) is accepted as a speaker reference too
     x = (np.random.RandomState(5).rand(4000).astype(np.float32) * 1.2 - 0.6)
     ours.TTSOutput(array=x, sample_rate=22050).save(tmp_path / "f32.wav")
     np.testing.assert_array_equal(load_audio(str(tmp_path / "f32.wav"), 22050), x)
 
 
-def test_randomised_requests_same_results(ref):
+def test_randomised_requests_same_results():
     """30 random (length, stream, failing chunk, scheduler concurrency) cases: both façades return the same audio in the same
     pieces, or fail with the same error."""
-    import importlib
-    from auralis_b200.base import ConditioningConfig as OursCC
-    RefCC = importlib.import_module("auralis.models.base").ConditioningConfig
     rng = np.random.RandomState(2024)
     for case in range(30):
         n_chars = int(rng.randint(1, 140))
@@ -230,24 +247,16 @@ def test_randomised_requests_same_results(ref):
         n_chunks = max(1, n_chars // 10)
         fail_at = int(rng.randint(n_chunks)) if rng.rand() < 0.25 else None
         conc = int(rng.choice([1, 2, 5, 16]))
-        results = []
-        for side in ("ref", "ours"):
-            if side == "ref":
-                tts = ref.TTS(scheduler_max_concurrency=conc); tts._ensure_event_loop()
-                tts.tts_engine = make_engine(ref.TTSOutput, RefCC(speaker_embeddings=True, gpt_like_decoder_conditioning=True), fail_at=fail_at)
-                Req = ref.TTSRequest
-            else:
-                tts = ours.TTS(scheduler_max_concurrency=conc).from_engine(make_engine(ours.TTSOutput, OursCC(True, True), fail_at=fail_at))
-                Req = ours.TTSRequest
+
+        def body(tts, Req):
             try:
                 out = tts.generate_speech(Req(text="r" * n_chars, speaker_files=["s.wav"], language="en", stream=stream))
                 if stream:
-                    got = ("ok", [np.asarray(c.array).tolist() for c in out])
-                else:
-                    got = ("ok", np.asarray(out.array).tolist())
+                    return ("ok", [np.asarray(c.array).tolist() for c in out])
+                return ("ok", np.asarray(out.array).tolist())
             except Exception as e:      # noqa: BLE001
-                got = ("err", type(e).__name__, str(e))
-            results.append(got)
+                return ("err", type(e).__name__, str(e))
+        results = _both(f"randomised[{case}]", body, conc=conc, fail_at=fail_at)
         if results[0][0] == "err" and stream:
             assert results[1][0] == "err" and results[1][1:] == results[0][1:], (case, results)
         else:

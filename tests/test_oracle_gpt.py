@@ -152,10 +152,15 @@ def _reference_penalizer():
 
 def test_repetition_penalty_matches_the_reference_class(dims_small):
     """hijack.py:49-88 — the reference's OWN penaliser, run as-is on the prompt the reference builds
-    (`[1]*(32+Lt)+[start]`, vllm_mm_gpt.py:325) plus a generated history with repeats."""
-    Pen = _reference_penalizer()
-    if Pen is None:
-        pytest.skip("reference tree not mounted")
+    (`[1]*(32+Lt)+[start]`, vllm_mm_gpt.py:325) plus a generated history with repeats.  What it changed is stored in
+    tests/golden/oracle_gpt_reference.npz (tests/reference_records.py)."""
+    from reference_records import Records
+    rec = Records("oracle_gpt_reference")
+
+    def reference(prompt, gen, z, p):
+        want = _reference_penalizer()(p)(prompt, gen, z.clone())
+        changed = torch.nonzero(want != z).reshape(-1)
+        return changed, want[changed]
     g = dims_small.gpt
     rng = np.random.RandomState(4)
     for trial in range(20):
@@ -166,7 +171,9 @@ def test_repetition_penalty_matches_the_reference_class(dims_small):
         gen = rng.randint(0, V, size=int(rng.randint(0, 30))).tolist()
         gen = gen + gen[:3]                                              # repeats must be penalised once
         p = [5.0, 1.0, 2.5, 0.5][trial % 4]
-        want = Pen(p)(prompt, gen, z.clone())
+        changed, values = rec(f"repetition_penalty[{trial}]", lambda: reference(prompt, gen, z, p))
+        want = z.clone()
+        want[torch.from_numpy(changed)] = torch.from_numpy(values)
         seen = O.prompt_seen_set(g) | set(gen)
         got = O.apply_repetition_penalty(z.clone(), seen, p)
         assert torch.equal(got, want), (trial, p)

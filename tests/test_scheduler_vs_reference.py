@@ -1,5 +1,6 @@
-"""CPU, container only: `auralis_b200.scheduler.TwoPhaseScheduler` against the REFERENCE's own scheduler
-(`common/scheduling/two_phase_scheduler.py`, imported unmodified by oracle/ref_sched.py), scenario by scenario, under the
+"""CPU: `auralis_b200.scheduler.TwoPhaseScheduler` against what the REFERENCE's own scheduler
+(`common/scheduling/two_phase_scheduler.py`, imported unmodified by oracle/ref_sched.py) did, stored in
+tests/golden/scheduler_vs_reference.npz (tests/reference_records.py), scenario by scenario, under the
 contract the XTTS engine uses it with — every phase-2 generator yields exactly one item (vLLM FINAL_ONLY, XTTSv2.py:738).
 Compared: the items and their order, the exception type and message that reach the caller, how many generators were ever
 in flight at once, and which ones were started first.
@@ -12,9 +13,9 @@ import asyncio
 import pytest
 
 from auralis_b200.scheduler import TwoPhaseScheduler as Ours
-from oracle import ref_import
+from reference_records import Records
 
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
+rec = Records("scheduler_vs_reference")
 
 
 async def _scenario(S, n=5, fail_at=None, conc=2, first_fails=False, slow_gen=None, sched_kw=None):
@@ -55,10 +56,13 @@ def _run(S, **kw):
     return asyncio.new_event_loop().run_until_complete(main())
 
 
-@pytest.fixture(scope="module")
-def Ref():
+def _ref_run(**kw):
     from oracle import ref_sched
-    return ref_sched.load()
+    return _run(ref_sched.load(), **kw)
+
+
+def _key(name, kw):
+    return name + "[" + ",".join(f"{k}={v}" for k, v in kw.items()) + "]"
 
 
 @pytest.mark.timeout(120)
@@ -66,8 +70,8 @@ def Ref():
     dict(n=1), dict(n=5), dict(n=7, conc=1), dict(n=7, conc=3), dict(n=4, conc=10),
     dict(n=5, fail_at=0), dict(n=5, fail_at=2), dict(n=5, fail_at=4), dict(n=3, first_fails=True),
 ], ids=lambda kw: ",".join(f"{k}={v}" for k, v in kw.items()))
-def test_same_behaviour_as_the_reference_scheduler(Ref, kw):
-    want = _run(Ref, **kw)
+def test_same_behaviour_as_the_reference_scheduler(kw):
+    want = rec(_key("scenario", kw), lambda: _ref_run(**kw))
     got = _run(Ours, **kw)
     assert (got[1] is None) == (want[1] is None)
     if want[1] is None:
@@ -82,9 +86,9 @@ def test_same_behaviour_as_the_reference_scheduler(Ref, kw):
 
 
 @pytest.mark.timeout(120)
-def test_timeouts_raise_timeout_error_like_the_reference(Ref):
+def test_timeouts_raise_timeout_error_like_the_reference():
     for kw in (dict(n=3, slow_gen=1, sched_kw=dict(request_timeout=0.15)), dict(n=3, slow_gen=1, sched_kw=dict(generator_timeout=0.15))):
-        want = _run(Ref, **kw)
+        want = rec(_key("timeout", kw), lambda: _ref_run(**kw))
         got = _run(Ours, **kw)
         assert want[1] is not None and got[1] is not None, (want, got)
         assert got[1][0] == want[1][0] == "TimeoutError", (want, got)

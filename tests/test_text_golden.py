@@ -9,7 +9,7 @@ import pytest
 
 from auralis_b200 import text as X
 from auralis_b200 import textnorm as T
-from oracle import ref_import, ref_text
+from oracle import ref_text
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "text_cleaners.json")
 
@@ -46,10 +46,12 @@ def test_golden_vectors_from_the_reference():
         assert ("expand_numbers_multilingual", lang) in seen and ("multilingual_cleaners", lang) in seen
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
 def test_live_against_the_reference_module():
+    """Random cleaner inputs and sentence splits; the reference tokenizer's answers are stored in
+    tests/golden/text_reference_fuzz.npz (tests/reference_records.py)."""
     import random
-    ref = ref_text.load()
+    from reference_records import Records
+    rec = Records("text_reference_fuzz")
     rng = random.Random(7)
     alphabet = "abc dr. mr. sr. st. co. 1 2 3 12 1.234 5,50 $ £ € % & # @ ° º ª th st er e . , ; ! ?".split(" ")
     for lang in ["en", "es", "fr", "de", "it", "pt", "pl", "ar", "zh", "cs", "ru", "nl", "tr", "hu", "ko"]:
@@ -57,13 +59,14 @@ def test_live_against_the_reference_module():
             s = " ".join(rng.choice(alphabet) for _ in range(rng.randint(1, 14)))
             if rng.random() < 0.5:
                 s = s.replace(" ", "", rng.randint(0, 4))
-            assert T.multilingual_cleaners(s, lang, n2w=ref_text.marker_num2words) == ref.multilingual_cleaners(s, lang), (lang, s)
+            want = rec(f"multilingual_cleaners[{lang}]{s}", lambda: ref_text.load().multilingual_cleaners(s, lang))
+            assert T.multilingual_cleaners(s, lang, n2w=ref_text.marker_num2words) == want, (lang, s)
     for _ in range(20):
         n = rng.randint(3, 30)
         s = " ".join(rng.choice(["Short one.", "A somewhat longer sentence, with a clause; and more - much more - to say about it all", "Why?",
                                  "Numbers like 1.5 do not end sentences.", "Ellipsis... then more!"]) for _ in range(n))
         lim = rng.choice([40, 82, 166, 250])
-        assert X.split_sentence(s, "en", lim) == ref.split_sentence(s, "en", lim)
+        assert X.split_sentence(s, "en", lim) == rec(f"split_sentence[{lim}]{s}", lambda: ref_text.load().split_sentence(s, "en", lim))
 
 
 def test_number_words_follow_num2words_conventions():

@@ -1,13 +1,11 @@
-"""CPU: the Chinese normaliser (auralis_b200/zh_textnorm.py) against the reference's own `zh_num2words` — golden records
-everywhere, live fuzz when /root/reference is mounted."""
+"""CPU: the Chinese normaliser (auralis_b200/zh_textnorm.py) against the reference's own `zh_num2words` — golden records,
+and a fuzz whose reference answers are stored in tests/golden/zh_textnorm_fuzz.npz (tests/reference_records.py)."""
 import json
 import os
 
-import pytest
-
 from auralis_b200 import textnorm as T
 from auralis_b200 import zh_textnorm as Z
-from oracle import ref_import
+from reference_records import Records
 from zh_fixture import load_reference_zh, sentences
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "zh_textnorm.json")
@@ -32,18 +30,18 @@ def test_examples():
     assert T.multilingual_cleaners("价格 5£ 和 3°, 共12个!", "zh") == "价格 五 英镑 和 三 度 , 共十二个,"
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
 def test_live_fuzz_against_the_reference_module():
-    z = load_reference_zh()
-    norm = z.TextNorm()
-    for s in sentences(3000, 99):
-        assert Z.normalize(s) == norm(s), s
-    ref_tok = None
-    try:
+    rec = Records("zh_textnorm_fuzz")
+    fuzz = sentences(3000, 99)
+    want = rec("TextNorm", lambda: [load_reference_zh().TextNorm()(s) for s in fuzz])
+    for s, w in zip(fuzz, want, strict=True):
+        assert Z.normalize(s) == w, s
+
+    def reference_cleaners(ss):
         from oracle import ref_text
         ref_tok = ref_text.load()
-    except Exception:
-        pass
-    if ref_tok is not None:                       # the whole zh cleaner chain of the reference tokenizer
-        for s in sentences(300, 7):
-            assert T.multilingual_cleaners(s, "zh") == ref_tok.multilingual_cleaners(s, "zh"), s
+        return [ref_tok.multilingual_cleaners(s, "zh") for s in ss]
+    fuzz = sentences(300, 7)                       # the whole zh cleaner chain of the reference tokenizer
+    want = rec("multilingual_cleaners", lambda: reference_cleaners(fuzz))
+    for s, w in zip(fuzz, want, strict=True):
+        assert T.multilingual_cleaners(s, "zh") == w, s
